@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- training_step throughput of the HashGrid + FullyFusedMLP hot path (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one trainer->training_step (fused fwd+loss+bwd kernel + Adam) over one batch of 2^18 synthetic
 uniform-[0,1)^3 positions with closed-form targets. Prints ONE JSON line (rank 0). See DESIGN.md "Measurement".
@@ -164,7 +164,6 @@ def run_reference(args):
             "config": config_dict(1, "dp1")}  # the reference is a single-GPU library: one GPU whatever --gpus says
     modes = {}
     if os.path.exists(harness):
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
         env = dict(os.environ)
         for name, cfg, jit in (("fully_fused", "headline.json", 0), ("fully_fused_jit", "headline.json", 1), ("cutlass", "headline_cutlass.json", 0)):
             cmd = [harness, "bench", os.path.join(ROOT, "tests", "golden", "configs", cfg), str(N_IN), str(N_OUT), str(BATCH), str(args.steps), str(args.warmup), str(jit)]
@@ -307,6 +306,14 @@ def run_own(args):
     prof = model.read_profile()
     model.set_profiling(False)
     launches = tcnn_b200.kernel_launch_count() - launches0
+    if args.dump_outputs:
+        # what a caller of the timed step receives after its last step: the loss of that step and the trained parameters
+        loss_last = dp.loss()
+        dp.sync_full_precision()
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "loss.npy"), np.array([loss_last], np.float64))
+            np.save(os.path.join(args.dump_outputs, "params.npy"), trainer.params_full_precision().cpu().numpy().astype(np.float32))
     # loss of training step number warmup + steps (one more step on the next batch of the pool): the reference arm prints the same
     # quantity after the same number of steps on the same data sequence (rank 0 draws the reference's pcg32{1337} stream)
     step(args.warmup + args.steps)
@@ -424,7 +431,10 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="own", choices=["own", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss and parameters after the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         run_reference(args)

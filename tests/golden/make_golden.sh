@@ -28,3 +28,11 @@ $H dump $C/identity_cutlass.json 3 3 512 10 "$OUT/identity_cutlass" 0
 $H dump $C/composite_nrc.json 6 3 512 10 "$OUT/composite_nrc" 0
 $H dump $C/composite_grid_sh.json 6 3 512 10 "$OUT/composite_grid_sh" 0
 $H dump $C/frequency_top.json 3 3 512 10 "$OUT/frequency_top" 0
+# Trainer::serialize() snapshots (msgpack), without and with the optimizer state, at initialisation and after 20 steps; a small
+# model keeps the fixture small
+for opt in 0 1; do
+	for steps in 0 20; do
+		mkdir -p "$OUT/snapshot_opt${opt}_step${steps}"
+		$H snapshot save $C/snapshot_small.json 3 3 1024 $steps "$OUT/snapshot_opt${opt}_step${steps}" $opt > "$OUT/snapshot_opt${opt}_step${steps}/save.json"
+	done
+done

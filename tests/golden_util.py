@@ -1,4 +1,5 @@
 """Loader for tests/golden/*.npz (vectors dumped from the unmodified reference on a B200, see tests/golden/make_golden.sh)."""
+import hashlib
 import json
 import os
 
@@ -33,6 +34,15 @@ def device_scales(name, n_levels):
     probe = json.load(open(os.path.join(GOLDEN, CASES[name][4])))
     bits = np.array([l["dev_bits"] for l in probe["levels"][:n_levels]], np.uint32)
     return bits.view(np.float32).tolist(), probe
+
+
+def init_params_match(g, params):
+    """Initial fp32 parameters bit for bit against the reference's: the stored array, or its SHA-256 where the fixture keeps only
+    the digest to stay small (tests/golden/pack_golden.py)."""
+    params = np.ascontiguousarray(params, np.float32)
+    if "params_init_f32" in g:
+        return np.array_equal(params.view(np.uint32), g["params_init_f32"].view(np.uint32))
+    return hashlib.sha256(params.tobytes()).hexdigest() == g["meta"]["params_init_sha256"]
 
 
 def rae(a, b, percentile=100.0):

@@ -107,20 +107,84 @@ def test_unmodified_reference_sample_trains(torch_cuda, tmp_path):
     assert os.path.getsize(tmp_path / "learned.jpg") > 1000 and os.path.exists(tmp_path / "reference.jpg")
 
 
+def msgpack_decode(b):
+    """The part of MessagePack that nlohmann::json::to_msgpack writes for a snapshot: maps, arrays, strings, binaries, numbers."""
+    import struct
+
+    def num(i, fmt):
+        n = struct.calcsize(fmt)
+        return struct.unpack(">" + fmt, b[i : i + n])[0], i + n
+
+    def seq(n, i, pairs):
+        out = {} if pairs else []
+        for _ in range(n):
+            if pairs:
+                k, i = val(i)
+                out[k], i = val(i)
+            else:
+                v, i = val(i)
+                out.append(v)
+        return out, i
+
+    def val(i):
+        t = b[i]
+        i += 1
+        if t <= 0x7F or t >= 0xE0:
+            return (t if t <= 0x7F else t - 256), i
+        if t <= 0x8F or 0x90 <= t <= 0x9F:
+            return seq(t & 0x0F, i, t <= 0x8F)
+        if 0xA0 <= t <= 0xBF:
+            return b[i : i + (t & 0x1F)].decode(), i + (t & 0x1F)
+        if t in (0xC0, 0xC2, 0xC3):
+            return {0xC0: None, 0xC2: False, 0xC3: True}[t], i
+        if t in (0xC4, 0xC5, 0xC6, 0xD9, 0xDA, 0xDB):
+            n, i = num(i, {0xC4: "B", 0xC5: "H", 0xC6: "I", 0xD9: "B", 0xDA: "H", 0xDB: "I"}[t])
+            return (bytes(b[i : i + n]) if t <= 0xC6 else b[i : i + n].decode()), i + n
+        if t in (0xDC, 0xDD, 0xDE, 0xDF):
+            n, i = num(i, "H" if t in (0xDC, 0xDE) else "I")
+            return seq(n, i, t >= 0xDE)
+        fmt = {0xCA: "f", 0xCB: "d", 0xCC: "B", 0xCD: "H", 0xCE: "I", 0xCF: "Q", 0xD0: "b", 0xD1: "h", 0xD2: "i", 0xD3: "q"}.get(t)
+        if fmt is None:
+            raise ValueError(f"msgpack type 0x{t:02x} is not part of a snapshot")
+        return num(i, fmt)
+
+    v, end = val(0)
+    assert end == len(b)
+    return v
+
+
+def snapshot_schema(v):
+    """Keys, value kinds and binary sizes of a decoded snapshot: what decides whether a reader accepts it."""
+    if isinstance(v, dict):
+        return {k: snapshot_schema(x) for k, x in v.items()}
+    if isinstance(v, bytes):
+        return ("bytes", len(v))
+    return type(v if not isinstance(v, float) else 0.0).__name__
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("with_optimizer", [0, 1])
 def test_snapshots_interoperate_with_the_reference(torch_cuda, tmp_path, with_optimizer):
-    """trainer->serialize() / deserialize() (trainer.h:442-482, optimizers/adam.h:303-325) exchange the reference's JSON schema: a
-    snapshot written by the UNMODIFIED reference (oracle/_ref/ref_harness, msgpack as instant-ngp stores it) loads into this library
-    and reproduces the reference's inference; a snapshot written by this library loads into the reference and reproduces ours."""
-    harness = os.path.join(ROOT, "oracle", "_ref", "ref_harness")
+    """trainer->serialize() / deserialize() (trainer.h:442-482, optimizers/adam.h:303-325) exchange the reference's JSON schema.
+    tests/golden/snapshot_small.npz holds snapshots the UNMODIFIED reference wrote (msgpack, as instant-ngp stores them) at
+    initialisation and after 20 steps, and its inference after the 20 steps. The 20-step snapshot loads into this library and
+    reproduces the reference's inference; the snapshot this library writes at initialisation decodes to exactly the reference's, and
+    the one it writes after 20 steps has the reference's keys, value kinds and sizes and loads back into this library."""
     exe = os.path.join(ROOT, "tests", "cpp", "snapshot_interop")
-    if not (os.path.exists(harness) and os.path.exists(exe)):
-        pytest.skip("oracle/_ref/ref_harness or tests/cpp/snapshot_interop has not been built")
-    cfg = os.path.join(ROOT, "tests", "golden", "configs", "hash3d_small.json")
+    if not os.path.exists(exe):
+        pytest.skip("tests/cpp/snapshot_interop has not been built")
+    from golden_util import GOLDEN, rae
+
+    g = np.load(os.path.join(GOLDEN, "snapshot_small.npz"))
+    meta = json.loads(bytes(g["meta"]).decode())
+    cfg = os.path.join(GOLDEN, "configs", "snapshot_small.json")
     env = dict(os.environ, LD_LIBRARY_PATH=os.path.join(ROOT, "tiny-cuda-nn_b200") + ":" + os.environ.get("LD_LIBRARY_PATH", ""))
     d = str(tmp_path)
-    B = 1024
+    B = str(meta["batch"])
+    g["x_f32"].tofile(os.path.join(d, "x.f32"))
+    g["y_f32"].tofile(os.path.join(d, "y.f32"))
+    ref0, ref20 = (g[f"snapshot_opt{with_optimizer}_step{n}"].tobytes() for n in (0, 20))
+    open(os.path.join(d, "snapshot.msgpack"), "wb").write(ref20)
 
     def run(cmd):
         out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env)
@@ -128,22 +192,23 @@ def test_snapshots_interoperate_with_the_reference(torch_cuda, tmp_path, with_op
         return json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
 
     # reference -> this library
-    saved = run([harness, "snapshot", "save", cfg, "3", "3", str(B), "20", d, str(with_optimizer)])
-    loaded = run([exe, "load", cfg, "3", "3", str(B), d, os.path.join(d, "snapshot.msgpack")])
-    ref = np.fromfile(os.path.join(d, "inference.f32"), np.float32)
+    loaded = run([exe, "load", cfg, "3", "3", B, d, os.path.join(d, "snapshot.msgpack")])
+    ref = g[f"inference_snapshot_opt{with_optimizer}_step20_f32"]
     ours = np.fromfile(os.path.join(d, "inference_loaded.f32"), np.float32)
-    from golden_util import rae
-
     assert rae(ours, ref, 99.0) < 1e-2  # same parameters, the two forward kernels (tests/test_common.h:177)
     assert loaded["has_optimizer"] == bool(with_optimizer)
     # the step after loading continues the reference's trajectory (with its optimizer state: moments + per-parameter step counters)
-    assert loaded["next_step_loss"] < 1.5 * saved["last_loss"] + 1e-6
-    # this library -> reference
-    run([exe, "save", cfg, "3", "3", str(B), d, "20", str(with_optimizer)])
-    back = run([harness, "snapshot", "load", cfg, "3", "3", str(B), d, os.path.join(d, "snapshot_b200.msgpack")])
+    assert loaded["next_step_loss"] < 1.5 * meta["last_loss"][f"snapshot_opt{with_optimizer}_step20"] + 1e-6
+    # this library -> reference: at initialisation the parameters are bit-exact with the reference's, so the whole snapshot must be
+    run([exe, "save", cfg, "3", "3", B, d, "0", str(with_optimizer)])
+    assert msgpack_decode(open(os.path.join(d, "snapshot_b200.msgpack"), "rb").read()) == msgpack_decode(ref0)
+    run([exe, "save", cfg, "3", "3", B, d, "20", str(with_optimizer)])
+    ours20 = open(os.path.join(d, "snapshot_b200.msgpack"), "rb").read()
+    assert snapshot_schema(msgpack_decode(ours20)) == snapshot_schema(msgpack_decode(ref20))
+    back = run([exe, "load", cfg, "3", "3", B, d, os.path.join(d, "snapshot_b200.msgpack")])
     ours2 = np.fromfile(os.path.join(d, "inference_b200.f32"), np.float32)
-    ref2 = np.fromfile(os.path.join(d, "inference_loaded.f32"), np.float32)
-    assert rae(ours2, ref2, 99.0) < 1e-2
+    back2 = np.fromfile(os.path.join(d, "inference_loaded.f32"), np.float32)
+    assert rae(back2, ours2, 99.0) < 1e-2
     assert np.isfinite(back["next_step_loss"])
 
 

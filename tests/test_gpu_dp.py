@@ -15,6 +15,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_data_parallel_engines_match_single_gpu(torch_cuda):
     torch = torch_cuda
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs at least 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "dp_parity.py")], capture_output=True, text=True, timeout=900)
     assert out.returncode == 0 and "DP PARITY OK" in out.stdout, out.stdout[-3000:] + out.stderr[-3000:]

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 import oracle_binding as ob
-from golden_util import CASES, device_scales, load_case, load_config, mlp_gradients_agree, rae
+from golden_util import CASES, device_scales, init_params_match, load_case, load_config, mlp_gradients_agree, rae
 
 h2f = ob.half_bits_to_float
 
@@ -39,7 +39,7 @@ def test_inputs_and_initial_parameters_bit_exact(case):
     m = ob.OracleModel(n_in, n_out, case["cfg"])
     assert m.n_params == g["meta"]["n_params"]
     assert m.grid.n_params == g["meta"]["n_encoding_params"]
-    assert np.array_equal(m.params_fp32.view(np.uint32), g["params_init_f32"].view(np.uint32))
+    assert init_params_match(g, m.params_fp32)
 
 
 def test_encoded_features_bit_exact(case):
@@ -81,6 +81,8 @@ def test_gradients_and_adam_within_reference_tolerances(case):
     g, n_in, n_out, B = case["g"], case["n_in"], case["n_out"], case["B"]
     x, y = g["x_f32"].reshape(B, n_in), g["y_f32"].reshape(B, n_out)
     m = ob.OracleModel(n_in, n_out, case["cfg"], accum_mode=ob.ACCUM_FP16_K16, scales=case["scales"])
+    p0 = m.params_fp32.copy()
+    assert init_params_match(g, p0)
     loss0 = m.training_step(x, y, run_optimizer=False)
     assert abs(loss0 - g["meta"]["losses"][0]) < 1e-3 * g["meta"]["losses"][0]
     grads = h2f(m.grads_fp16)
@@ -95,8 +97,8 @@ def test_gradients_and_adam_within_reference_tolerances(case):
     loss1 = m.training_step(x, y)
     p1 = g["params_step1_f32"]
     lr = case["cfg"]["optimizer"]["learning_rate"]
-    moved_ref = p1 != g["params_init_f32"]
-    moved = m.params_fp32 != g["params_init_f32"]
+    moved_ref = p1 != p0
+    moved = m.params_fp32 != p0
     assert (moved != moved_ref).mean() < 2e-3  # zero-gradient skip (adam.h:79-82)
     # first Adam step = lr * sign(g) (bias-corrected m/sqrt(v)), so parameters agree to ~1e-3 * lr except where a tiny
     # gradient changes sign between implementations
